@@ -35,6 +35,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the tree may be read-only: nothing is written there, not even __pycache__
 sys.path.insert(0, ROOT)
 
 READ_LEN = 150
@@ -70,6 +71,8 @@ def parse_args():
     ap.add_argument("--no-cli-crosscheck", action="store_true")
     ap.add_argument("--repeat-frac", type=float, default=float(os.environ.get("SNAPGPU_BENCH_REPEAT_FRAC", "0")),
                     help="SURVEY 8d stress variant: this fraction of the reference is drawn from a 10 kbp repeat library at 0-5 %% divergence")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the headline's result records of the last timed step (rank 0) as DIR/<field>.npy")
     return ap.parse_args()
 
 
@@ -242,10 +245,28 @@ def to_host_batch(dev_batch, pinned=True):
     return synth.ReadBatch(rb.cpu().numpy(), rq.cpu().numpy(), ro.cpu().numpy().astype(np.uint64), rl.cpu().numpy().astype(np.uint32))
 
 
-def run_workload(c, args, name, batches, W, K, sample_clocks=False):
+DUMP_LIMIT = 64 * 10**6                 # bytes of all the .npy files --dump-outputs writes
+
+
+def dump_outputs(d, records):
+    """The result records a caller of the timed path receives, one float64 array per field (paired fields are [pairs, 2]), as d/<field>.npy.
+    When all rows would not fit in DUMP_LIMIT bytes, a fixed sample of rows (seed 0, ascending) is written, with its row numbers as
+    d/rows.npy; the inputs are seeded, so two builds run with the same arguments can be compared array for array."""
+    names = [f for f in records.dtype.names if f != "reserved"]
+    row_bytes = 8 + sum(8 * int(np.prod(records.dtype[f].shape)) for f in names)
+    n = len(records)
+    m = min(n, (DUMP_LIMIT - (1 << 16)) // row_bytes)           # 64 KiB left for the .npy headers
+    rows = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "rows.npy"), rows.astype(np.float64))
+    for f in names:
+        np.save(os.path.join(d, f + ".npy"), records[f][rows].astype(np.float64))
+
+
+def run_workload(c, args, name, batches, W, K, sample_clocks=False, dump_dir=None):
     """One workload on this rank (all ranks call it together): device-resident timing over exactly K steps after W warm-ups, then the
     same through the C ABI with host buffers.  Returns the workload's object; ["_records"] holds the engine's records for batches[0]
-    (rank 0, for the parity leg), ["_host0"] those reads on the host."""
+    (rank 0, for the parity leg), ["_host0"] those reads on the host.  dump_dir: where rank 0 writes the records of the last timed step."""
     import torch
     import torch.distributed as dist
     from snap_b200 import engine, shard
@@ -265,7 +286,7 @@ def run_workload(c, args, name, batches, W, K, sample_clocks=False):
     # them are recorded on the same stream (a NULL stream argument would mean "the aligner's own stream")
     stream = torch.cuda.Stream(device)
     assert stream.cuda_stream != 0
-    res = torch.empty((n_units, res_dtype.itemsize), dtype=torch.uint8, device=device)
+    res = torch.zeros((n_units, res_dtype.itemsize), dtype=torch.uint8, device=device)
     d_ctr = torch.zeros((engine.N_COUNTERS,), dtype=torch.int64, device=device)
 
     def step(b):
@@ -299,6 +320,8 @@ def run_workload(c, args, name, batches, W, K, sample_clocks=False):
     launches = al.launch_count() - launches0
     if paired:
         al.check(stream.cuda_stream)        # raises if a kernel latched an error (pool overflow)
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, res.cpu().numpy().view(res_dtype).reshape(-1))
     ctr = d_ctr.cpu().numpy()
     ms_max = shard.max_over_ranks(ms_total, device) if world > 1 else ms_total
     ctr_all = shard.allreduce_counters(ctr, device) if world > 1 else ctr
@@ -1009,7 +1032,7 @@ def run_ours(args):
     batches = {kind: make_batches(c, args, kind, W + K)}
     torch.cuda.synchronize()
     c.setup["reads_s"] = round(time.time() - t0, 2)
-    head = run_workload(c, args, headline, batches[kind], W, K, sample_clocks=True)
+    head = run_workload(c, args, headline, batches[kind], W, K, sample_clocks=True, dump_dir=args.dump_outputs)
     clocks = head.pop("_clocks")
 
     # ---- the other BASELINE configs, each to the same bar (device-resident + e2e + roofline; parity below): configs[2] / [4] paired,
@@ -1164,6 +1187,8 @@ def main():
     os.dup2(2, 1)                      # C-level stdout of this process (and its children) -> stderr
     sys.stdout = sys.stderr
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs writes the engine's records; it does not apply to --impl reference")
         run_reference(args)
     else:
         run_ours(args)

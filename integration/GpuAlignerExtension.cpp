@@ -7,7 +7,7 @@
  *
  * This file is the ONLY code that touches SNAP types; below it everything is plain C (pointers, sizes, POD structs).  It is
  * compiled against the reference headers where they lie and linked with the UNMODIFIED SNAPLib objects and -lsnapgpu by
- * integration/Makefile.  Must compile as C++98 like the reference.
+ * oracle/Makefile.  Must compile as C++98 like the reference.
  *
  * Threading contract (the reference: one BaseAligner per worker thread, "NOT thread safe", BaseAligner.h:19-20).  A GPU aligner
  * handle owns tens of GB of per-warp arenas, so it is NOT per SNAP thread: there is ONE engine (index image + one single-end

@@ -14,11 +14,13 @@ import json
 import os
 import shutil
 import subprocess
+import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(os.path.dirname(HERE), "snap_b200", "csrc")
 LIB = os.path.join(CSRC, "libsnapgpu.so")
-CACHE = LIB + ".stamp.json"
+# cached outside the tree (bench.py may run from a read-only checkout), one file per library path
+CACHE = os.path.join(tempfile.gettempdir(), "snapgpu_sass_stamps_%s.json" % hashlib.sha256(LIB.encode()).hexdigest()[:16])
 
 # workload key prefix in traffic.json -> substring of the (mangled) names of the kernels its capture holds
 GROUPS = {"single": "sg_align_kernel", "ag_d20": "sg_align_kernel", "ne_d20": "sg_align_kernel", "paired": "sg_align_paired_kernel",
@@ -42,7 +44,7 @@ def _cuobjdump():
 
 def sass_stamps():
     """{kernel-name substring: sha16 of the SASS of every kernel whose name holds it} for the built library; {} when there is no
-    cuobjdump or no library.  Cached beside the library (keyed by its size and mtime)."""
+    cuobjdump or no library.  Cached in CACHE (keyed by the library's size and mtime)."""
     if not os.path.exists(LIB):
         return {}
     st = os.stat(LIB)

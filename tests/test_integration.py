@@ -1,4 +1,4 @@
-"""The compiled drop-in: integration/_build/snap-aligner-gpu = the UNMODIFIED reference (SNAPLib objects) linked with
+"""The compiled drop-in: oracle/_ref/snap-aligner-gpu = the UNMODIFIED reference (SNAPLib objects) linked with
 integration/GpuAlignerExtension.cpp and libsnapgpu.so.  `snap-aligner-gpu single|paired <index> reads.fq -o out.sam` must write the
 records stock `snap-aligner` writes for the same command line -- the reference's own option parser, FASTQ reader, filter and SAM
 writer run on both sides; only the aligner behind AlignerExtension::runIterationThread differs."""
@@ -10,14 +10,14 @@ import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-GPU_BIN = os.path.join(ROOT, "integration", "_build", "snap-aligner-gpu")
+GPU_BIN = os.path.join(ROOT, "oracle", "_ref", "snap-aligner-gpu")
 
 
 def test_binding_is_built_and_links_the_product_library():
-    """CPU-side: the binary exists (built by __graft_entry__.build() where /root/reference is present) and its only non-system
+    """CPU-side: the binary exists (built by __graft_entry__.build() where the reference sources are present) and its only non-system
     dependency is libsnapgpu.so; no compute here."""
     if not os.path.exists(GPU_BIN):
-        pytest.skip("integration/_build/snap-aligner-gpu not built (needs /root/reference once: make -C integration)")
+        pytest.skip("oracle/_ref/snap-aligner-gpu not built (needs the reference sources once: make -C oracle ref)")
     out = subprocess.run(["ldd", GPU_BIN], capture_output=True, text=True).stdout
     assert "libsnapgpu.so" in out and "not found" not in out, out
     assert "libsnapref" not in out            # the oracle shim is not part of the drop-in
@@ -51,7 +51,7 @@ def _stats_line(stdout, n=5):
 @pytest.mark.parametrize("threads", [1, 4])
 def test_snap_aligner_gpu_single_writes_the_stock_records(tmp_path, small_cfg, reflib, threads):
     if not os.path.exists(GPU_BIN):
-        pytest.fail("integration/_build/snap-aligner-gpu is missing on the GPU box")
+        pytest.fail("oracle/_ref/snap-aligner-gpu is missing")
     from snap_b200 import synth
     reads = small_cfg.reads["noisy150"]           # N runs, short reads, noise, indels
     fq = str(tmp_path / "r.fq")
@@ -102,7 +102,7 @@ def test_snap_aligner_gpu_single_secondary_alignments(tmp_path, small_cfg, refli
 @pytest.mark.parametrize("threads", [1, 3])
 def test_snap_aligner_gpu_paired_writes_the_stock_records(tmp_path, small_cfg, reflib, threads):
     if not os.path.exists(GPU_BIN):
-        pytest.fail("integration/_build/snap-aligner-gpu is missing on the GPU box")
+        pytest.fail("oracle/_ref/snap-aligner-gpu is missing")
     pairs = small_cfg.pairs["std150"]             # chimeric mates, N runs, short ends
     f1, f2 = str(tmp_path / "r1.fq"), str(tmp_path / "r2.fq")
     with open(f1, "wb") as a, open(f2, "wb") as b:

@@ -11,7 +11,7 @@ from conftest import OPTION_SETS, differing
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-GPU_BIN = os.path.join(ROOT, "integration", "_build", "snap-aligner-gpu")
+GPU_BIN = os.path.join(ROOT, "oracle", "_ref", "snap-aligner-gpu")
 
 
 @pytest.fixture(scope="module")
